@@ -6,6 +6,7 @@
   python bench.py --impl reference ...                      (the CPU port of the reference path on the host cores)
 
   python bench.py --variant C5|C3|C4 ...                    (the sibling configurations of BASELINE.json; C2 is the headline)
+  python bench.py --dump-outputs DIR ...                    (also write the last timed step's outputs as DIR/*.npy)
 
 One JSON line on rank 0. `value`: device-resident inputs, fwd + loss + bwd + grad all-reduce + clip + AdamW, timed with
 CUDA events, max over ranks. `e2e`: the same step through model.train_step with pinned HOST inputs (H2D inside the timed
@@ -77,7 +78,11 @@ def parse():
     ap.add_argument('--torch-profile', default='', help='write a torch.profiler kernel table of 2 steps to this path')
     ap.add_argument('--row-order', default=None, choices=['input', 'morton'],
                     help='row order of the sparse tensors (default: ESB200_ROW_ORDER or input); morton = Z-ordered rows')
+    ap.add_argument('--dump-outputs', default='', metavar='DIR',
+                    help='after the timed steps, write what the last timed step computed as DIR/<name>.npy (dump_outputs)')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs records the timed esb200 path; the reference arm times a different step')
     for k, v in VARIANTS[args.variant].items():
         if k in ('batch', 'views', 'height', 'width', 'points') and getattr(args, k) is None:
             setattr(args, k, v)
@@ -139,6 +144,34 @@ class ClockSampler:
         sm = sorted(self.sm)
         return {'sm_mhz': sm[len(sm) // 2], 'sm_max_mhz': self.max_mhz, 'reasons': sorted(self.reasons_seen),
                 'samples': len(sm), 'source': 'nvml' if self.nv is not None else 'nvidia-smi'}
+
+
+class InitialState:
+    """The seeded weights and buffers (BatchNorm statistics) a run starts from. fp32 atomics make the training trajectory
+    differ from run to run in the last bits, and AdamW and the head's top-k selections amplify that over tens of steps;
+    putting this state back before the step whose outputs are dumped gives that step's forward pass identical inputs in
+    every run. Restoring is a few launches, enqueued between two steps."""
+
+    def __init__(self, model, arena):
+        self.arena = arena
+        self.flat = arena.flat.clone()
+        self.bufs = list(model.buffers())
+        self.saved = [b.clone() for b in self.bufs]
+
+    def restore(self):
+        self.arena.flat.copy_(self.flat)
+        torch._foreach_copy_(self.bufs, self.saved)
+        self.arena.refresh_bf16()
+
+
+def dump_outputs(out_dir, logs):
+    """What the last timed train step computed, for comparing two builds output for output on the same seeded inputs
+    (the step starts from InitialState): every value train_step returned to its caller, as `<name>.npy` (float64
+    scalar). The weights the step leaves behind are not dumped: AdamW moves each of them by about lr with the sign of its
+    gradient, so wherever a gradient is within round-off of zero two runs of one build already differ."""
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in logs.items():
+        np.save(os.path.join(out_dir, k.replace(os.sep, '_') + '.npy'), np.asarray(float(v), dtype=np.float64))
 
 
 def _trainable(k, v):
@@ -291,6 +324,7 @@ def main():
     model = MODELS.build(dict(cfg, compute_dtype=dtype)).to(dev).train()
     optim = OptimWrapper(model, max_run_ahead=args.run_ahead, **opt)
     broadcast_parameters(optim.arena)
+    initial = InitialState(model, optim.arena) if args.dump_outputs else None
 
     n_distinct = 2
     batches = []
@@ -388,6 +422,8 @@ def main():
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for j in range(args.steps):
+        if initial is not None and j == args.steps - 1:
+            initial.restore()
         logs = step(args.warmup + j)
         if j in sample_at:
             ts = time.perf_counter()
@@ -402,6 +438,9 @@ def main():
     if prof_range:
         torch.cuda.profiler.stop()
     log('timed region done')
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, logs)
+        log(f'outputs of timed step {args.steps - 1} written to {args.dump_outputs}')
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -604,7 +604,40 @@ def gen_metrics():
          occupancy_json=np.array(json.dumps({k: float(v) for k, v in ret_occ.items()}, sort_keys=True)))
 
 
-GENERATORS = dict(metrics=gen_metrics, continuous_occ=gen_continuous_occ, continuous=gen_continuous, augment=gen_augment, grounding=gen_grounding, detector=gen_detector, occupancy=gen_occupancy, frontend=gen_frontend, functions=gen_functions,
+DROPIN_CONFIGS = ('configs/detection/mv-det3d_8xb4_embodiedscan-3d-284class-9dof.py',
+                  'configs/detection/cont-det3d_8xb1_embodiedscan-3d-284class-9dof.py',
+                  'configs/occupancy/mv-occ_8xb1_embodiedscan-occ-80class.py',
+                  'configs/occupancy/cont-occ_8xb1_embodiedscan-occ-80class.py',
+                  'configs/grounding/mv-grounding_8xb12_embodiedscan-vg-9dof.py',
+                  'configs/grounding/mv-grounding_8xb12_embodiedscan-vg-9dof_fcaf-coder.py')
+
+
+def gen_dropin():
+    """The drop-in boundary (registry.register_into_reference): the `model = dict(...)` of six unmodified config files,
+    stored as Python literals so tuples survive, and the names the reference's own MODELS / TASK_UTILS registries hold
+    once `embodiedscan.models` is imported. Written as dropin.json."""
+    import ast
+    import json
+
+    import embodiedscan
+    import embodiedscan.models  # noqa: F401  (registers the reference's classes)
+    from embodiedscan.registry import MODELS, TASK_UTILS
+    root = os.path.dirname(os.path.abspath(list(embodiedscan.__path__)[0]))
+    configs = {}
+    for f in DROPIN_CONFIGS:
+        scope = {}
+        exec(compile(open(os.path.join(root, f)).read(), f, 'exec'), scope)     # `_base_` files hold runtime settings only
+        configs[f] = repr(scope['model'])
+        assert ast.literal_eval(configs[f]) == scope['model'], f
+    path = os.path.join(HERE, 'dropin.json')
+    with open(path, 'w') as fh:
+        json.dump(dict(models=sorted(MODELS._m), task_utils=sorted(TASK_UTILS._m), configs=configs), fh, indent=1,
+                  sort_keys=True)
+        fh.write('\n')
+    print(f'wrote {path}: {os.path.getsize(path) / 1024:.1f} KiB')
+
+
+GENERATORS = dict(dropin=gen_dropin, metrics=gen_metrics, continuous_occ=gen_continuous_occ, continuous=gen_continuous, augment=gen_augment, grounding=gen_grounding, detector=gen_detector, occupancy=gen_occupancy, frontend=gen_frontend, functions=gen_functions,
                   eval=gen_eval)
 
 if __name__ == '__main__':

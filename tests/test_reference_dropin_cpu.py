@@ -1,21 +1,38 @@
-"""Drop-in check against the reference tree itself (dev container only: skipped where /root/reference is absent, e.g. on
-the GPU box). With the third-party stand-ins of tests/golden/refstubs.py installed, `register_into_reference()` must make
-the reference's OWN registry build the esb200 classes from the reference's UNMODIFIED config files."""
+"""Drop-in check of the registry boundary: `register_into_reference()` must make the reference's OWN registries build the
+esb200 classes from the reference's UNMODIFIED config files. tests/golden/dropin.json (make_golden.py dropin) holds the
+`model` dicts of those config files and the names the reference's registries hold once its models are imported; the
+registries are rebuilt here as `embodiedscan/registry.py` defines them, every one of those names already taken, so the
+test needs neither the reference tree nor its third-party stack."""
+import ast
+import json
 import os
 import sys
+import types
 
 import pytest
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'embodiedscan')), reason='needs /root/reference')
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+with open(os.path.join(GOLD, 'dropin.json')) as _f:
+    DROPIN = json.load(_f)
 
 
-def load_config(path):
-    """The `model = dict(...)` of an mmengine python config (plain exec; `_base_` files only hold runtime settings)."""
-    scope = {}
-    exec(compile(open(path).read(), path, 'exec'), scope)
-    return scope['model']
+def reference_registry_module(monkeypatch):
+    """`embodiedscan.registry`: MODELS and TASK_UTILS as children of mmengine's roots (the mmengine stand-in of
+    refstubs.py), each holding a class of the reference under every name the reference registers."""
+    if GOLD not in sys.path:
+        sys.path.insert(0, GOLD)
+    from refstubs import Registry
+    mod = types.ModuleType('embodiedscan.registry')
+    for attr, key in (('MODELS', 'models'), ('TASK_UTILS', 'task_utils')):
+        reg = Registry(attr.lower(), parent=Registry(attr.lower()))
+        for name in DROPIN[key]:
+            reg.register_module(module=type(name, (), {'__module__': 'embodiedscan.models'}))
+        setattr(mod, attr, reg)
+    pkg = types.ModuleType('embodiedscan')
+    pkg.__path__, pkg.registry = [], mod
+    monkeypatch.setitem(sys.modules, 'embodiedscan', pkg)
+    monkeypatch.setitem(sys.modules, 'embodiedscan.registry', mod)
+    return mod
 
 
 @pytest.mark.parametrize('cfg_file,cls_name', [
@@ -26,23 +43,19 @@ def load_config(path):
     ('configs/grounding/mv-grounding_8xb12_embodiedscan-vg-9dof.py', 'SparseFeatureFusion3DGrounder'),
     ('configs/grounding/mv-grounding_8xb12_embodiedscan-vg-9dof_fcaf-coder.py', 'SparseFeatureFusion3DGrounder'),
 ])
-def test_reference_registry_builds_esb200_from_unmodified_configs(cfg_file, cls_name):
-    if GOLD not in sys.path:
-        sys.path.insert(0, GOLD)
-    import refstubs
-    refstubs.install(REF)
-    import embodiedscan.models  # noqa: F401  (the reference registers its own classes first)
-    from embodiedscan.registry import MODELS as REF_MODELS
+def test_reference_registry_builds_esb200_from_unmodified_configs(cfg_file, cls_name, monkeypatch):
+    ref = reference_registry_module(monkeypatch)
+    assert cls_name in DROPIN['models']                   # the reference's own class holds the name until the override
 
     import embodiedscan_b200
     from embodiedscan_b200.registry import register_into_reference
     register_into_reference()
-    model_cfg = load_config(os.path.join(REF, cfg_file))
+    model_cfg = ast.literal_eval(DROPIN['configs'][cfg_file])
     assert model_cfg['type'] == cls_name
     for sub in ('backbone', 'neck'):                      # pretrained-checkpoint URLs need a network
         if isinstance(model_cfg.get(sub), dict):
             model_cfg[sub].pop('init_cfg', None)
-    model = REF_MODELS.build(model_cfg)
+    model = ref.MODELS.build(model_cfg)
     assert type(model).__module__.startswith('embodiedscan_b200'), type(model)
     assert type(model) is getattr(embodiedscan_b200, cls_name, None) or type(model).__name__ == cls_name
     names = dict(model.named_parameters())
